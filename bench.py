@@ -79,6 +79,31 @@ class ClockSampler(threading.Thread):
             'samples': len(sm)}
 
 
+def model_state(model):
+  """Everything a training step reads and updates: parameters, Adam slots, normaliser state, step counters."""
+  v = model.variables
+  return ([t.clone() for t in (v.flat, v.adam_m, v.adam_v, v.state, v.state_snapshot, model._counters)],
+          (v.adam_t, model.flags.global_step, model._counters_mirror))
+
+
+def restore_model_state(model, saved):
+  v = model.variables
+  with torch.no_grad():
+    for dst, src in zip((v.flat, v.adam_m, v.adam_v, v.state, v.state_snapshot, model._counters), saved[0]):
+      dst.copy_(src)
+  v.adam_t, model.flags.global_step, model._counters_mirror = saved[1]
+  if v.weight_table is not None:
+    v.weight_table.dirty = True      # the step rebuilds the weight planes from the restored parameters
+
+
+def step_outputs(model, losses):
+  """What one training step hands its caller, as float32 host arrays: the two returned losses and the step's named
+  losses (GanModel.last_losses)."""
+  out = {'generator_loss': losses[0], 'discriminator_loss': losses[1]}
+  out.update({'loss_' + k: t for k, t in model.last_losses.items() if k not in out})
+  return {k: t.detach().to('cpu', torch.float32).reshape(-1).numpy() for k, t in out.items()}
+
+
 def bench_cuda(args):
   import torch.distributed as dist
   from twingan_b200 import ops, twingan, flops
@@ -123,6 +148,10 @@ def bench_cuda(args):
     # pre-flight: N NCCL ranks == N sequential micro-batches through the product, parameters identical across ranks
     from twingan_b200 import ddp
     ddp_check = ddp.selfcheck(dev, pg)
+  # --dump-outputs: the last timed step starts again from the seeded initial state.  Steps are reproducible only to fp32
+  # rounding (atomics order in split-K / wgrad reductions) and training amplifies that from step to step, so without the
+  # reset what the last step computes would differ from run to run.  The reset is one copy inside the timed window.
+  initial_state = model_state(model) if args.dump_outputs else None
   use_graph = not args.no_graph
   if use_graph:
     model.capture(*dev_inputs[0])
@@ -161,9 +190,13 @@ def bench_cuda(args):
   e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
   e0.record()
   for i in range(args.steps):
-    step_resident(i)
+    if initial_state is not None and i == args.steps - 1:
+      restore_model_state(model, initial_state)
+    last = step_resident(i)
   e1.record()
   barrier()
+  # copied now: the legs below run further steps on the same model
+  dumped = step_outputs(model, last) if args.dump_outputs and rank == 0 else None
   launches = (L.launch_count() - launches0) if not use_graph else model.launches_per_step * args.steps
   ms = e0.elapsed_time(e1)
   # e2e leg
@@ -271,6 +304,13 @@ def bench_cuda(args):
         out['secondary'] = {'infer': {'error': repr(e)}}
     if not args.no_cpu_baseline and world == 1:
       out['cpu_baseline'] = cpu_baseline_subprocess(args)
+    if dumped is not None:
+      import numpy as np
+      os.makedirs(args.dump_outputs, exist_ok=True)
+      for k, a in dumped.items():
+        np.save(os.path.join(args.dump_outputs, k + '.npy'), a)
+      out['dumped_outputs'] = {'dir': args.dump_outputs, 'arrays': len(dumped),
+                               'bytes': sum(a.nbytes for a in dumped.values())}
     print(json.dumps(out), flush=True)
   if world > 1:
     dist.destroy_process_group()
@@ -508,7 +548,14 @@ def main():
   ap.add_argument('--profile-one-step', action='store_true', help='1 warm-up + 1 step only (for ncu launch lists)')
   ap.add_argument('--no-secondary', action='store_true', help='skip the configs[4] inference measurement (secondary.infer)')
   ap.add_argument('--no-ddp-check', action='store_true', help='skip the data-parallel pre-flight at N > 1')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='write the losses the last timed training step returned as DIR/<name>.npy; that step starts from '
+                       'the seeded initial model state and its inputs are seeded, so two builds compare output for output')
   args = ap.parse_args()
+  if args.dump_outputs and (args.impl != 'cuda' or args.workload != 'train' or args.profile_one_step):
+    ap.error('--dump-outputs writes the outputs of the timed training step: --impl cuda --workload train only')
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
   if args.impl == 'reference':
     bench_reference(args)
     return

@@ -1,17 +1,17 @@
 """Golden vectors produced by THE REFERENCE'S OWN network code.
 
-Runs /root/reference/nets/pggan.py (+ nets/pggan_utils.py, libs/batch_norm.py, libs/instance_norm.py and the leaky-ReLU
+Runs the reference's nets/pggan.py (+ nets/pggan_utils.py, libs/batch_norm.py, libs/instance_norm.py and the leaky-ReLU
 of util_misc.py:68-86) under tests/golden/tf18_shim.py -- a torch-backed stand-in for the few dozen TensorFlow-1.8 API
 entry points those files use -- with the wiring of twingan.py:196-270,370-373 (scopes `encoder_content`, `generator`,
 `discriminator_s`; per-domain `_s` / `_t` normaliser postfixes; UNet end points), and stores inputs, every variable the
 reference created (under the name the reference gave it), outputs, end points, gradients and the normaliser state after
-the pass in tests/golden/reference_pggan.npz.
+the pass in tests/golden/reference_pggan.npz, in the compact form of tests/golden/golden_store.py (seeded inputs as
+their seeds, large result tensors as statistics plus a fixed sample of elements).
 
-Only runnable where /root/reference exists (this authoring container); the .npz travels.  tests/test_cpu_reference_golden.py
-then holds oracle/twingan_oracle.py to these vectors.  What this does and does not pin is stated at the top of
-tf18_shim.py.
+Needs a checkout of the reference (jerryli27/TwinGAN); the .npz files do not.  tests/test_cpu_reference_golden.py then holds
+oracle/twingan_oracle.py to these vectors.  What this does and does not pin is stated at the top of tf18_shim.py.
 
-  python tests/golden/make_reference_golden.py [--reference /root/reference]
+  python tests/golden/make_reference_golden.py --reference <TwinGAN checkout> [--f4]
 """
 from __future__ import annotations
 
@@ -29,6 +29,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 import tf18_shim as tfs  # noqa: E402
+import golden_store  # noqa: E402
 from golden_provider import stable_hash_provider  # noqa: E402
 
 CASES = [
@@ -69,6 +70,11 @@ def load_reference(ref_root):
   import nets.pggan as pggan          # noqa: E402  (the reference)
   pggan_utils = pggan.pggan_utils
   return tf, pggan, pggan_utils
+
+
+def _stream(name, seed, draws):
+  """The draws of one case's seeded generator, in order: tests/golden/golden_store.py replays them instead of storing them."""
+  return np.array(json.dumps({'seed': seed, 'draws': [['%s/%s' % (name, k), kind, list(shape)] for k, kind, shape in draws]}))
 
 
 def run_case(tf, pggan, pggan_utils, case, out):
@@ -120,7 +126,9 @@ def run_case(tf, pggan, pggan_utils, case, out):
 
   # a scalar functional of everything, for gradients (fixed random cotangents)
   L = 0.0
+  draws = [('in/sources', 'rand', sources.t.shape), ('in/targets', 'rand', targets.t.shape)]
   for k, v in outs:
+    draws.append(('cot/' + k, 'randn', v.t.shape))
     cot = torch.randn(v.t.shape, generator=g, dtype=torch.float64)
     out[name + '/cot/' + k] = cot.numpy()
     L = L + (v.t * cot).sum()
@@ -129,6 +137,7 @@ def run_case(tf, pggan, pggan_utils, case, out):
   f32 = lambda t: t.detach().to(torch.float32).numpy()
   out[name + '/in/sources'] = sources.t.detach().numpy()
   out[name + '/in/targets'] = targets.t.detach().numpy()
+  out[name + '/rng_stream'] = _stream(name, 100 + hw, draws)
   provider = stable_hash_provider(1)
   for n, v in tfs.STORE.vars.items():
     if v.trainable:
@@ -304,6 +313,9 @@ def run_clone_case(tf, pggan, GanModel, ns, case, out):
   out[name + '/random_log'] = np.array([str(r) for r in tfs.STORE.random_log])
   for key, d in zip(draw_keys, draws):
     out[name + '/uniform01/' + key] = d.numpy()
+  out[name + '/rng_stream'] = _stream(name, 500 + hw, [('in/sources', 'rand', sources.t.shape),
+                                                       ('in/targets', 'rand', targets.t.shape)] +
+                                      [('uniform01/' + k, 'rand', d.shape) for k, d in zip(draw_keys, draws)])
   out[name + '/extra_flags'] = np.array(json.dumps(extra, sort_keys=True))
   out[name + '/var_order'] = np.array(list(tfs.STORE.vars.keys()))
   out[name + '/var_trainable'] = np.array([bool(v.trainable) for v in tfs.STORE.vars.values()])
@@ -401,6 +413,11 @@ def run_deploy_case(tf, pggan, GanModel, ns, out, name='deploy2_in8', hw=8, mc=1
     out[name + '/in/targets_%d' % c] = batches[c]['b_source'].t.detach().numpy()
     for j, key in enumerate(('alpha_s', 'noise_s', 'alpha_t', 'noise_t')):
       out[name + '/uniform01/%s_%d' % (key, c)] = draws[4 * c + j].numpy()
+  out[name + '/rng_stream'] = _stream(name, 900, [
+      d for c in range(2) for d in [('in/sources_%d' % c, 'rand', batches[c]['a_source'].t.shape),
+                                    ('in/targets_%d' % c, 'rand', batches[c]['b_source'].t.shape)] +
+      [('uniform01/%s_%d' % (key, c), 'rand', draws[4 * c + j].shape)
+       for j, key in enumerate(('alpha_s', 'noise_s', 'alpha_t', 'noise_t'))]])
   out[name + '/var_order'] = np.array([n for n, v in tfs.STORE.vars.items() if v.trainable])
   out[name + '/var_shapes'] = np.array([str(list(v.t.shape)) for n, v in tfs.STORE.vars.items() if v.trainable])
   out[name + '/generator_loss'] = np.array(float(g_loss.t))
@@ -466,7 +483,7 @@ def reference_stage_loop(ref_root, tf, flag_values):
 
 def main():
   ap = argparse.ArgumentParser()
-  ap.add_argument('--reference', default='/root/reference')
+  ap.add_argument('--reference', required=True, help='checkout of the reference project (jerryli27/TwinGAN)')
   ap.add_argument('--out', default=os.path.join(HERE, 'reference_pggan.npz'))
   ap.add_argument('--f4', action='store_true', help='only the SURVEY 8f-4 optional-flag cases -> reference_f4.npz')
   args = ap.parse_args()
@@ -477,7 +494,7 @@ def main():
     for case in F4_CLONE_CASES:
       run_clone_case(tf, pggan, GanModel, ns, case, out)
     path = os.path.join(os.path.dirname(args.out), 'reference_f4.npz')
-    np.savez_compressed(path, **out)
+    golden_store.save(path, out)
     print('wrote %s (%.1f MB, %d arrays)' % (path, os.path.getsize(path) / 1e6, len(out)))
     return
   for case in CASES:
@@ -486,7 +503,7 @@ def main():
   for case in CLONE_CASES:
     run_clone_case(tf, pggan, GanModel, ns, case, out)
   run_deploy_case(tf, pggan, GanModel, ns, out)
-  np.savez_compressed(args.out, **out)
+  golden_store.save(args.out, out)
   import json
   meta = {'flag_defaults': reference_flag_defaults(args.reference)}
   for tag, fl in (('default', dict(train_dir='/ckpt', is_training=True, do_export=False, program_name='twingan',

@@ -8,7 +8,8 @@ recipe's full 256x256 / 256-channel size too), layer order, which layers carry n
 pixel-norm, the fade-in lerps, UNet end-point selection, minibatch-stddev, the normalisers' forward arithmetic, their
 stop-gradients (through the gradients) and their moving-average pushes.  TensorFlow's own kernels (conv2d, avg_pool,
 nearest-neighbour resize, moments, batch_normalization, slim's layer wrappers) are restated in the stand-in and stay
-unpinned (DESIGN.md 4)."""
+unpinned (DESIGN.md 4).  The files keep large result tensors as a sample plus whole-tensor statistics and the seeded inputs
+as their seeds (tests/golden/golden_store.py)."""
 import ast
 import os
 import sys
@@ -19,6 +20,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, 'golden'))
+import golden_store  # noqa: E402
 from golden_provider import stable_hash_provider  # noqa: E402
 from oracle import twingan_oracle as O  # noqa: E402
 
@@ -29,7 +31,7 @@ NAME_CASES = ['full256', 'full128grow']
 
 @pytest.fixture(scope='module')
 def golden():
-  return np.load(GOLDEN)
+  return golden_store.load(GOLDEN)
 
 
 def _cfg(z, case):
@@ -39,6 +41,8 @@ def _cfg(z, case):
 
 
 def _rel(a, b):
+  if isinstance(b, golden_store.Sample):
+    return b.rel(a)
   a, b = torch.as_tensor(a, dtype=torch.float64), torch.as_tensor(b, dtype=torch.float64)
   return float((a - b).abs().max() / b.abs().max().clamp_min(1e-300))
 
@@ -165,7 +169,7 @@ F4_CASES = ['f4_wgan_gp8', 'f4_wgan8', 'f4_hinge16grow', 'f4_gan8', 'f4_eqlr_dra
 
 @pytest.fixture(scope='module')
 def golden_f4():
-  return np.load(os.path.join(HERE, 'golden', 'reference_f4.npz'))
+  return golden_store.load(os.path.join(HERE, 'golden', 'reference_f4.npz'))
 
 
 @pytest.mark.parametrize('case', F4_CASES)
@@ -285,7 +289,7 @@ def _check_whole_clone(z, case):
       assert float(grads[n].abs().max()) == 0.0, n
     else:
       ref = z['%s/grad/%s' % (case, n)]
-      if float(np.abs(ref).max()) < 1e-12:
+      if (ref.absmax if isinstance(ref, golden_store.Sample) else float(np.abs(ref).max())) < 1e-12:
         # mathematically zero on both sides (e.g. a residual shortcut's bias in front of a 1x1 conv + instance norm): only
         # rounding residue is left to compare
         assert float(grads[n].abs().max()) < 1e-12, n

@@ -205,20 +205,23 @@ def test_graph_replay_matches_eager(built_lib):
                                   'f4_res_eqlr_renorm8'])
 def test_product_matches_vectors_from_the_reference_code(built_lib, case):
   """The CUDA path against tests/golden/reference_pggan.npz directly: losses and forward tensors that the reference's own
-  _clone_fn / add_loss produced under the TF stand-in (tests/golden/make_reference_golden.py).  Forward quantities
-  only -- gradient parity needs the kink-aware comparison of test_step_parity."""
+  _clone_fn / add_loss produced under the TF stand-in (tests/golden/make_reference_golden.py; large tensors are kept as a
+  sample, tests/golden/golden_store.py).  Forward quantities only -- gradient parity needs the kink-aware comparison of
+  test_step_parity."""
   import ast
   import os
   import sys
   import numpy as np
   here = os.path.dirname(os.path.abspath(__file__))
   sys.path.insert(0, os.path.join(here, 'golden'))
+  import golden_store
   from golden_provider import stable_hash_provider
   from oracle import twingan_oracle as O
   from twingan_b200 import ops, twingan
   from tests.parity import rel_err
   import json
-  z = np.load(os.path.join(here, 'golden', 'reference_f4.npz' if case.startswith('f4_') else 'reference_pggan.npz'))
+  z = golden_store.load(os.path.join(here, 'golden', 'reference_f4.npz' if case.startswith('f4_') else 'reference_pggan.npz'))
+  ref_err = lambda mine, ref: ref.rel(mine) if isinstance(ref, golden_store.Sample) else rel_err(mine, torch.as_tensor(ref))
   hw, growing, mc, batch, gs, max_steps = [int(v) for v in z[case + '/meta']]
   norm = str(z[case + '/norm'])
   alpha = (gs / max_steps) if growing else 0.0
@@ -256,10 +259,10 @@ def test_product_matches_vectors_from_the_reference_code(built_lib, case):
                           ('discriminator_real_s_prediction', 'pred_real_s'),
                           ('discriminator_s_prime_prediction', 'pred_s_prime'),
                           ('discriminator_t_cycle_prediction', 'pred_t_cycle')):
-      assert rel_err(ends[mine], torch.as_tensor(z['%s/ep/%s' % (case, ref_key)])) < REL_TOL, (case, prec, ref_key)
+      assert ref_err(ends[mine], z['%s/ep/%s' % (case, ref_key)]) < REL_TOL, (case, prec, ref_key)
     # the inference tensor of the same graph (inference/image_translation_infer.py:46-99): eval-mode E(.;'_s') -> G(.;'_t')
     translated = model.infer(f32(z[case + '/in/sources']))
-    assert rel_err(translated, torch.as_tensor(z[case + '/infer/custom_generated_t_style_source'])) < REL_TOL, (case, prec)
+    assert ref_err(translated, z[case + '/infer/custom_generated_t_style_source']) < REL_TOL, (case, prec)
   ops.set_precision(1)
 
 
