@@ -586,7 +586,9 @@ class InferencePipeline(object):
   copy of batch k+1 and the device->host copy of result k-1 run on side streams while batch k computes; the device
   staging slots and the pinned result slots are allocated once and reused across `run` calls.
   `use_graph`: the ~90 kernel launches of a batch are captured once per batch shape into a CUDA graph over a static input
-  buffer and replayed (the weights are read through the persistent weight-plane table, so a later `load_dict` is seen)."""
+  buffer and replayed.  The tensor-core convs of the graph read the weights through the persistent weight-plane table,
+  which the replay cannot rebuild by itself: `_infer` refreshes the table first when the variables changed since it was
+  last built (`load_dict`, `init_random`), so a replay after a reload translates with the new weights."""
 
   def __init__(self, model: GanModel, depth: int = 2, use_graph: bool = False):
     from .prefetch import HostReturner
@@ -618,6 +620,9 @@ class InferencePipeline(object):
       self._graphs[key] = ent
     graph, static_in, static_out = ent
     static_in.copy_(x, non_blocking=True)
+    table = self.model.variables.weight_table
+    if table is not None and table.dirty:
+      table.refresh()            # variables changed since the capture (load_dict, init): the graph reads these planes
     graph.replay()
     return static_out.clone()                           # the static buffer is overwritten by the next replay
 
